@@ -2,7 +2,7 @@
 """
 bench.py -- env-steps/sec of the B200-native batched simulator (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload kuka|mobile] [--no-secondary]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload kuka|mobile] [--no-secondary] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -25,6 +25,8 @@ rl_baselines/rl_algorithm/ppo2.py:58-72): a single kernel launch, 4096 x 128 env
                  ppo2_config3     = configs[2], PPO2 from rl_baselines.train on 4096 Kuka envs, 14 updates (rank 0)
   --impl reference : the reference arm.  PyBullet is not installable here, so it times the oracle -- the CPU
           restatement of the reference's step -- with every host thread, on the same configs.
+  --dump-outputs DIR : after the timed steps, write what the headline rollout returned in the last timed step (rank 0's envs) as
+          DIR/<name>.npy, so that two builds run with the same arguments can be compared output for output (see dump_outputs).
 """
 import argparse
 import hashlib
@@ -154,6 +156,26 @@ def make_inputs(workload, n, T, seed):
         noise = rng.normal(0, 0.01, (T, n)).astype(np.float32)
         return acts, noise
     return rng.integers(0, 4, (T, n), dtype=np.int32), None
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+DUMP_SAMPLE_SEED = 12345
+
+
+def dump_outputs(outdir, arrays):
+    """Write host arrays laid out [T, n, ...] as <outdir>/<name>.npy.  float32 stays float32; integer outputs become float64, which holds
+    them exactly.  When the arrays exceed DUMP_BUDGET_BYTES together, every one keeps the same env columns, a sample drawn from a fixed
+    seed, so the files of two runs with the same arguments cover the same envs."""
+    def out_dtype(a):
+        return np.float32 if a.dtype == np.float32 else np.float64
+    n = next(iter(arrays.values())).shape[1]
+    total = sum(a.size * np.dtype(out_dtype(a)).itemsize for a in arrays.values())
+    if total > DUMP_BUDGET_BYTES:
+        cols = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(n, n * DUMP_BUDGET_BYTES // total, replace=False))
+        arrays = {k: a[:, cols] for k, a in arrays.items()}
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.ascontiguousarray(a, dtype=out_dtype(a)))
 
 
 def workload_spec(workload):
@@ -467,10 +489,13 @@ def run_reference(args):
         for _ in range(warmup):
             pool.step()
         times = [pool.step() for _ in range(steps)]
-        return n, T, pool.threads, sum(times)
+        return n, T, pool.threads, sum(times), pool
 
     spec = workload_spec(args.workload)
-    n, T, threads, total = run(args.workload, args.steps, args.warmup)
+    n, T, threads, total, pool = run(args.workload, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {name: np.concatenate([p[k] for p in pool.parts], axis=1)
+                                         for name, k in (("obs", 3), ("reward", 4), ("done", 5))})
     value = n * T * args.steps / total
     sample = ("%d envs x %d steps per step, %d host threads (container CPU quota; %d CPUs visible), CPU oracle "
               "(PyBullet itself is not installable offline)" % (n, T, threads, os.cpu_count() or 1))
@@ -490,7 +515,7 @@ def run_reference(args):
             "e2e": {"value": value, "unit": "env-steps/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     if not args.no_secondary and args.workload == "kuka":
         sec = {}
-        mn, mT, mth, mtot = run("mobile", 3, 1)
+        mn, mT, mth, mtot, _ = run("mobile", 3, 1)
         sec["mobile_config4"] = {"metric": metric_and_config("mobile", 1)[0], "value": mn * mT * 3 / mtot, "unit": "env-steps/s", "cores": mth,
                                  "sample": "%d envs x %d steps per step x 3 (bounded sample of the T=1024 rollout), CPU oracle" % (mn, mT)}
         sec["plumbing_config1"] = plumbing_config1(_oracle_library(), -1)
@@ -504,8 +529,9 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------------- GPU arm -------------
-def measure_b200(be, workload, args, rank, world, local_rank, dist, sampler_holder):
-    """Device-timed and end-to-end throughput of one workload on this rank's GPU; max over ranks.  Returns a dict on every rank."""
+def measure_b200(be, workload, args, rank, world, local_rank, dist, sampler_holder, dump_dir=None):
+    """Device-timed and end-to-end throughput of one workload on this rank's GPU; max over ranks.  Returns a dict on every rank.
+    With `dump_dir`, rank 0 writes the outputs of the last timed rollout there (dump_outputs)."""
     import torch
     spec = workload_spec(workload)
     n, T, D = spec["n"], spec["T"], spec["obs_dim"]
@@ -551,6 +577,9 @@ def measure_b200(be, workload, args, rank, world, local_rank, dist, sampler_hold
         ev[k][1].record()
     barrier()
     wall = time.perf_counter() - wall0
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"obs": be.to_host(obs), "reward": be.to_host(rew), "done": be.to_host(done),
+                                "episode_return": be.to_host(ep_ret), "episode_length": be.to_host(ep_len)})
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = sum(step_ms)
     launches = sim.launch_count - launches0
@@ -624,7 +653,7 @@ def run_b200(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     be = Backend(load_cuda_library(), local_rank)
-    main = measure_b200(be, args.workload, args, rank, world, local_rank, dist, None)
+    main = measure_b200(be, args.workload, args, rank, world, local_rank, dist, None, dump_dir=args.dump_outputs)
     secondary = {}
     if not args.no_secondary and args.workload == "kuka":
         m = measure_b200(be, "mobile", args, rank, world, local_rank, dist, None)
@@ -679,6 +708,8 @@ def main():
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the configs[3] / configs[0] legs (A/B scripts, ncu captures)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)
