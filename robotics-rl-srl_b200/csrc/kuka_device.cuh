@@ -621,6 +621,9 @@ KK_DEV void kuka_dynamics(const KukaParams& P, const KukaEnv& e, const KukaKin& 
 
 #endif
 // In-place: M (lower) -> A = M^-1 (lower triangle valid), via Cholesky and triangular inverse.
+// Every loop has a constant trip count and skips the indices outside the triangle with an `if` that folds once the enclosing loops are
+// unrolled.  With bounds that depend on an outer index (i = j + 1 .. n) the compiler unrolls the inner loops before the outer ones, cannot
+// unroll them fully, and M drops to a 576-byte local-memory array (a local load / store per entry in the once-per-step code).
 KK_DEV void kuka_spd_inverse(float (&M)[KK_NB][KK_NB]) {
     constexpr int n = KK_NB;
     float dinv[n];
@@ -628,15 +631,18 @@ KK_DEV void kuka_spd_inverse(float (&M)[KK_NB][KK_NB]) {
     for (int j = 0; j < n; ++j) {
         float d = M[j][j];
 #pragma unroll
-        for (int kk = 0; kk < j; ++kk) d = fmaf(-M[j][kk], M[j][kk], d);
+        for (int kk = 0; kk < n; ++kk)
+            if (kk < j) d = fmaf(-M[j][kk], M[j][kk], d);
         const float inv = rsqrtf(d);
         dinv[j] = inv;
         M[j][j] = d * inv;
 #pragma unroll
-        for (int i = j + 1; i < n; ++i) {
+        for (int i = 0; i < n; ++i) {
+            if (i <= j) continue;
             float s = M[i][j];
 #pragma unroll
-            for (int kk = 0; kk < j; ++kk) s = fmaf(-M[i][kk], M[j][kk], s);
+            for (int kk = 0; kk < n; ++kk)
+                if (kk < j) s = fmaf(-M[i][kk], M[j][kk], s);
             M[i][j] = s * inv;
         }
     }
@@ -645,10 +651,12 @@ KK_DEV void kuka_spd_inverse(float (&M)[KK_NB][KK_NB]) {
     for (int j = 0; j < n; ++j) {
         M[j][j] = dinv[j];
 #pragma unroll
-        for (int i = j + 1; i < n; ++i) {
+        for (int i = 0; i < n; ++i) {
+            if (i <= j) continue;
             float s = 0.f;
 #pragma unroll
-            for (int kk = j; kk < i; ++kk) s = fmaf(M[i][kk], M[kk][j], s);
+            for (int kk = 0; kk < n; ++kk)
+                if (kk >= j && kk < i) s = fmaf(M[i][kk], M[kk][j], s);
             M[i][j] = -s * dinv[i];
         }
     }
@@ -656,10 +664,12 @@ KK_DEV void kuka_spd_inverse(float (&M)[KK_NB][KK_NB]) {
 #pragma unroll
     for (int i = 0; i < n; ++i) {
 #pragma unroll
-        for (int j = 0; j <= i; ++j) {
+        for (int j = 0; j < n; ++j) {
+            if (j > i) continue;
             float s = 0.f;
 #pragma unroll
-            for (int kk = i; kk < n; ++kk) s = fmaf(M[kk][i], M[kk][j], s);
+            for (int kk = 0; kk < n; ++kk)
+                if (kk >= i) s = fmaf(M[kk][i], M[kk][j], s);
             M[i][j] = s;
         }
     }
@@ -702,14 +712,15 @@ KK_DEV void kuka_physics_step(const KukaParams& P, KukaEnv& e, const KukaKin& k,
         kc_dynamics(sc, P, e.qd, u, gmask);
 #endif
 #pragma unroll
-        for (int i = 0; i < KK_NB; ++i) {
-            bias[i] = sc[KC_OFF_BIAS + i];
+        for (int i = 0; i < KK_NB; ++i)
 #pragma unroll
             for (int j = 0; j <= i; ++j) A[i][j] = sc[KC_OFF_MA + i * KC_MS + j];
-        }
         // Cholesky + M^-1 in registers, by every lane: dealt to the 4 lanes through shared memory it was three times slower (12 dependent
         // pivot steps of load -> rsqrt -> scale -> store -> barrier; measured on B200, profiles/r02_kuka_coop_by_function.txt)
         kuka_spd_inverse(A);
+        // the bias stays in the scratch area until the inverse is done: the Cholesky does not need it
+#pragma unroll
+        for (int i = 0; i < KK_NB; ++i) bias[i] = sc[KC_OFF_BIAS + i];
     } else {
 #if KK_ROLL_DYN
     {
